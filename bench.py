@@ -22,6 +22,10 @@ source and what the CPU oracle reads: builder, judge and oracle see identical bi
 After the headline measurement the same process measures the other BASELINE.json configs (`extra_configs`: config 2,
 config 4's batch and config 5's shard shape with streaming epochs), each with its own recall check and roofline.
 
+`--dump-outputs DIR` saves the headline search's answer from its last timed step (scores and corpus rows, one row per
+query).  The corpus and the queries come from fixed seeds, so two builds run with the same arguments can be compared
+answer for answer.
+
 `--impl reference` times the CPU arm instead: the numpy brute-force oracle (BASELINE.md section 4) with all host
 threads on a bounded sample of the same workload.  It never touches the GPU engine.
 
@@ -88,7 +92,15 @@ def parse_args():
     ap.add_argument("--extra", default="cfg2,cfg4,cfg5", help="which extra configs to run")
     ap.add_argument("--data", default="numpy", choices=["numpy", "philox"],
                     help="philox: device generator for chunks >= 1 (quick profiling runs only; chunk 0 stays canonical)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline search's answer from its last timed step to DIR/scores.npy (float32) and "
+                         "DIR/indices.npy (float64), one row per query, for comparing two builds on the same inputs")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def bits_to_f32(bits):
@@ -98,6 +110,15 @@ def bits_to_f32(bits):
 
 def workload_name(rows, dim, batch, k):
     return f"{rows}x{dim} bf16 corpus, batch {batch}, top-{k}, cosine"
+
+
+def dump_outputs(directory, out):
+    """Save (score, index) as search() returned them: cosine scores as float32, corpus rows as float64 (exact for every
+    row index)."""
+    os.makedirs(directory, exist_ok=True)
+    scores, indices = (x.cpu().numpy() for x in out)
+    np.save(os.path.join(directory, "scores.npy"), scores.astype(np.float32))
+    np.save(os.path.join(directory, "indices.npy"), indices.astype(np.float64))
 
 
 def measured_peaks():
@@ -923,6 +944,8 @@ def run_b200(a):
     wl = Workload(a, env, ix, sh, host, n_total, n_local, lo_row, dim, B, k, q_bits,
                   workload_name(n_total, dim, B, k))
     m, out, res_host, ms_total, nb_total = wl.measure(a.steps, a.warmup, a.min_timed_s, a.preheat_max, sampler)
+    if a.dump_outputs and rank == 0:           # every rank ends with the same merged answer
+        dump_outputs(a.dump_outputs, out)
     result = None
     if rank == 0:
         data_note = (f"synthetic, canonical numpy PCG64 (oracle.synth_rows seed {a.seed} per 262144-row chunk, rows not "

@@ -141,6 +141,27 @@ def test_reference_arm_prints_the_contract_line():
     assert out1.returncode == 0 and out1.stdout.strip() == ""
 
 
+def test_dump_outputs_saves_the_answer_as_float_arrays(tmp_path):
+    """--dump-outputs: what search() returned, scores as float32 and corpus rows as float64 holding the exact rows."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    s = torch.tensor([[0.75, 0.5], [1.0, -1.0]], dtype=torch.float32)
+    i = torch.tensor([[9_999_999, 0], [3, 2**31 - 1]], dtype=torch.int32)
+    bench.dump_outputs(str(tmp_path / "out"), (s, i))
+    scores, indices = np.load(tmp_path / "out" / "scores.npy"), np.load(tmp_path / "out" / "indices.npy")
+    assert scores.dtype == np.float32 and (scores == s.numpy()).all()
+    assert indices.dtype == np.float64 and (indices == i.numpy()).all()
+    assert sorted(os.listdir(tmp_path / "out")) == ["indices.npy", "scores.npy"]
+
+
+def test_bench_rejects_arguments_it_cannot_honour(tmp_path):
+    for args in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                             timeout=120)
+        assert out.returncode == 2 and out.stdout == "", args
+
+
 def test_harness_and_tool_scripts_compile():
     """The GPU harness can only run on a B200 box; at least keep it syntactically alive here."""
     import glob
